@@ -5,6 +5,7 @@ configs/two_head_model.yaml, 64 x 30 s synthetic 44.1 kHz mono clips per GPU, bf
 
     python bench.py --gpus N --steps K --warmup W            # this repo (libsome_b200.so kernels)
     python bench.py --impl reference ...                     # the reference algorithm on the host CPU cores
+    python bench.py ... --dump-outputs DIR                   # also write the last timed step's outputs as DIR/<name>.npy
 
 A "step" = one pass of the hot path over one batch (64 clips x 30 s = 1920 audio-seconds per GPU; weak
 scaling: each rank owns its own 64 clips, the only exchange is one all-gather of the packed notes).
@@ -62,6 +63,42 @@ def make_clips(first_index, count, seconds):
         base = pool[gi % len(pool)]
         clips.append(np.ascontiguousarray(np.roll(base, 4099 * (gi // len(pool))) * np.float32(1.0 - 0.01 * (gi % 7))))
     return clips
+
+
+DUMP_BYTES = 64 * 10 ** 6 - 2 ** 16            # --dump-outputs: 64 MB in all, with room for the .npy headers
+
+
+def dump_outputs(out_dir, arrays, seed=0):
+    """Writes each array as out_dir/<name>.npy, DUMP_BYTES in all.  The arrays are written smallest first and each may use an
+    equal share of the bytes left; a larger one is cut to a fixed, seeded sample of its rows, and <name>_rows.npy holds the
+    indices of the rows kept.  Same shapes -> same sample, so two builds can be compared output for output."""
+    os.makedirs(out_dir, exist_ok=True)
+    left = DUMP_BYTES
+    items = sorted(arrays.items(), key=lambda kv: kv[1].nbytes)
+    for i, (name, a) in enumerate(items):
+        share = left // (len(items) - i)
+        if a.nbytes > share:
+            keep = share // (a.nbytes // len(a) + 8)                # + the float64 row index
+            rows = np.sort(np.random.default_rng(seed).choice(len(a), keep, replace=False))
+            np.save(os.path.join(out_dir, f'{name}_rows.npy'), rows.astype(np.float64))
+            a = a[rows]
+            left -= rows.size * 8
+        np.save(os.path.join(out_dir, f'{name}.npy'), a)
+        left -= a.nbytes
+
+
+def device_step_outputs(eng, ws, m, cu, note_count):
+    """What one device step hands its caller, on the host: the head outputs of every frame and the decoded notes in the
+    layout of the note buffers (clip j's notes in rows cu[j] .. cu[j] + note_count[j] - 1, zero beyond), with durations in
+    seconds as Engine.infer returns them.  The shapes depend on the inputs only."""
+    count = note_count.cpu().numpy().astype(np.int64)
+    frames = np.diff(cu)
+    used = np.arange(m) - np.repeat(cu[:-1], frames) < np.repeat(count, frames)
+    return {'probs': ws.probs[:m].cpu().numpy(), 'bounds': ws.bounds[:m].cpu().numpy(),
+            'note_count': count.astype(np.float64),
+            'note_midi': np.where(used, ws.note_midi[:m].cpu().numpy(), 0).astype(np.float32),
+            'note_dur': np.where(used, ws.note_dur[:m].cpu().numpy() * eng.timestep, 0).astype(np.float64),
+            'note_rest': np.where(used, ws.note_rest[:m].cpu().numpy(), 0).astype(np.float32)}
 
 
 class ClockSampler:
@@ -196,9 +233,11 @@ def _pinned(clips):
     return out
 
 
-def measure_batch(ins, config_name, clips_per_gpu, seconds, steps, warmup, rank, world, dev, full, sampler=None):
+def measure_batch(ins, config_name, clips_per_gpu, seconds, steps, warmup, rank, world, dev, full, sampler=None,
+                  dump_dir=None):
     """Device-resident value, end-to-end value and per-kernel roofline of one (config, batch) on this rank; `full` adds the
-    pageable-input variant, the e2e breakdown, the strong-scaling figure and the parity check of the headline line."""
+    pageable-input variant, the e2e breakdown, the strong-scaling figure and the parity check of the headline line.
+    `dump_dir`: write the outputs of the last timed device step there (dump_outputs)."""
     import torch.distributed as dist
     from some_b200 import dist as sdist
     eng = ins.model
@@ -239,6 +278,8 @@ def measure_batch(ins, config_name, clips_per_gpu, seconds, steps, warmup, rank,
     barrier()
     dev_ms = ev0.elapsed_time(ev1)
     launches = eng.launches - launches0
+    if dump_dir is not None:
+        dump_outputs(dump_dir, device_step_outputs(eng, ws, m, cu, note_count))
     # second pass of the same K steps with CUDA events around every launch (recorded by the sequencer itself) for the roofline
     eng.start_profile(cu)
     barrier()
@@ -453,7 +494,8 @@ def run_ours(args, rank, world, local_rank):
     ins = build_plugin(args.config, local_rank)
     eng = ins.model
     sampler = ClockSampler(local_rank) if rank == 0 else None
-    meas = measure_batch(ins, args.config, args.clips, args.seconds, args.steps, args.warmup, rank, world, dev, True, sampler)
+    meas = measure_batch(ins, args.config, args.clips, args.seconds, args.steps, args.warmup, rank, world, dev, True, sampler,
+                         args.dump_outputs if rank == 0 else None)
     s = summarise(meas, args.steps, world, peaks)
 
     extra = {}
@@ -550,7 +592,13 @@ def main():
     ap.add_argument('--config', default='two_head', choices=['two_head', 'quant_two_head', 'midi_conformer'])
     ap.add_argument('--clips', type=int, default=64, help='clips per GPU')
     ap.add_argument('--seconds', type=float, default=30.0, help='clip length')
+    ap.add_argument('--dump-outputs', metavar='DIR',
+                    help='after the timed steps, write the outputs of the last one (rank 0: probs, bounds, notes) as DIR/<name>.npy')
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error('--steps must be at least 1')
+    if args.dump_outputs and args.impl != 'ours':
+        ap.error('--dump-outputs writes the outputs of this project\'s path (--impl ours)')
     rank = int(os.environ.get('RANK', '0'))
     world = int(os.environ.get('WORLD_SIZE', '1'))
     local_rank = int(os.environ.get('LOCAL_RANK', '0'))

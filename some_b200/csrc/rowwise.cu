@@ -145,15 +145,16 @@ __global__ void __launch_bounds__(256) row_stats_kernel(const RowStatsParams p) 
   }
 }
 
-// K-colmeans (calibration only, load time): column means of a GEMM's (effective) A operand.  One thread per column, rows
-// strided over blockIdx.y, partial sums combined with atomics into a zeroed buffer; the caller divides by M.
-__global__ void __launch_bounds__(128)
+// K-colmeans (calibration only, load time): column means of a GEMM's (effective) A operand.  A block owns 128 columns; its
+// 8 thread rows stride over the rows and their partial sums are added in a fixed order, so the means (and the bias
+// corrections derived from them) are the same in every run.
+__global__ void __launch_bounds__(128 * 8)
 col_means_kernel(const __nv_bfloat16* __restrict__ a, int M, int K, int lda, const float* __restrict__ stats, int parts,
                  float inv_m, float* __restrict__ out) {
+  __shared__ float part[8][128];
   const int k = blockIdx.x * 128 + threadIdx.x;
-  if (k >= K) return;
   float acc = 0.f;
-  for (int row = blockIdx.y; row < M; row += gridDim.y) {
+  for (int row = threadIdx.y; row < M && k < K; row += 8) {
     float v = __bfloat162float(a[(size_t)row * lda + k]);
     if (stats != nullptr) {
       float s = 0.f, q = 0.f;
@@ -165,7 +166,14 @@ col_means_kernel(const __nv_bfloat16* __restrict__ a, int M, int K, int lda, con
     }
     acc += v;
   }
-  atomicAdd(out + k, acc * inv_m);
+  part[threadIdx.y][threadIdx.x] = acc;
+  __syncthreads();
+  if (threadIdx.y == 0 && k < K) {
+    float s = 0.f;
+#pragma unroll
+    for (int i = 0; i < 8; ++i) s += part[i][threadIdx.x];
+    out[k] = s * inv_m;
+  }
 }
 
 __global__ void __launch_bounds__(256)
@@ -338,11 +346,8 @@ extern "C" int some_col_means(const uint16_t* a, int M, int K, int lda, const fl
                               cudaStream_t stream) {
   SOME_REQUIRE(a != nullptr && out != nullptr && M > 0 && K > 0 && K <= SOME_CALIB_K, "some_col_means: bad arguments");
   SOME_REQUIRE(ln_stats == nullptr || (ln_parts >= 1 && ln_parts <= SOME_LN_SLOTS), "some_col_means: bad ln_parts");
-  cudaError_t e = cudaMemsetAsync(out, 0, sizeof(float) * K, stream);
-  SOME_REQUIRE(e == cudaSuccess, "some_col_means: %s", cudaGetErrorString(e));
-  dim3 grid((K + 127) / 128, M < 64 ? M : 64);
-  col_means_kernel<<<grid, 128, 0, stream>>>(reinterpret_cast<const __nv_bfloat16*>(a), M, K, lda, ln_stats, ln_parts,
-                                             1.0f / M, out);
+  col_means_kernel<<<(K + 127) / 128, dim3(128, 8), 0, stream>>>(reinterpret_cast<const __nv_bfloat16*>(a), M, K, lda,
+                                                                  ln_stats, ln_parts, 1.0f / M, out);
   return check_launch("some_col_means");
 }
 

@@ -228,6 +228,32 @@ def test_row_stats(lib):
         torch.testing.assert_close(st[i][:, 0, 1], (x[i] * x[i]).sum(1), atol=1e-2, rtol=1e-5)
 
 
+@pytest.mark.parametrize('normalised', [False, True])
+def test_col_means(lib, normalised):
+    """some_col_means (load-time bias calibration): column means of a bf16 operand with a row pitch, optionally of the rows
+    normalised by LayerNorm statistics split over two slots, against float64 torch; bit-identical from launch to launch."""
+    torch.manual_seed(41)
+    m, k, lda = 1003, 2048, 2048 + 64
+    a = (torch.randn(m, lda, device=DEV) * 2 - 0.3).to(torch.bfloat16)
+    x = a[:, :k].double()
+    stats = None
+    if normalised:
+        stats = torch.zeros(m, _lib.LN_SLOTS, 2, device=DEV)
+        for s, cols in enumerate((slice(0, k // 2), slice(k // 2, k))):
+            stats[:, s, 0] = a[:, cols].float().sum(1)
+            stats[:, s, 1] = (a[:, cols].float() ** 2).sum(1)
+        mean = x.mean(1, keepdim=True)
+        x = (x - mean) * torch.rsqrt((x * x).mean(1, keepdim=True) - mean * mean + 1e-5)
+    outs = []
+    for _ in range(2):
+        out = torch.full((k,), float('nan'), device=DEV)
+        _lib.check(lib.some_col_means(a.data_ptr(), m, k, lda, _lib.ptr(stats), 2, out.data_ptr(), stream()), 'some_col_means')
+        outs.append(out)
+    torch.cuda.synchronize()
+    assert torch.equal(outs[0], outs[1])
+    torch.testing.assert_close(outs[0].double(), x.mean(0), atol=1e-6, rtol=1e-5)      # fp32 sums of 1003 O(1) values
+
+
 @pytest.mark.parametrize('n,epi', [(128, 'sigmoid'), (129, 'softmax'), (128, 'logits'), (129, 'logits')])
 def test_gemm_heads(lib, n, epi):
     torch.manual_seed(4)

@@ -1,6 +1,7 @@
 """CPU-only tests of the host logic: the C-ABI library loads and exports every symbol the header declares,
 config flattening / strict checkpoint schema, weight packing (GLU interleave, BN folding, mel tables),
 clip sharding + the gloo all-gather of note records (world_size 2), and the drop-in package alias."""
+import json
 import os
 import pathlib
 import re
@@ -108,11 +109,16 @@ def test_flatten_config_chain(tmp_path):
     assert flat == {'a': 2, 'd': {'x': 1, 'y': 3, 'z': 4}, 'keep': 7}
 
 
-@pytest.mark.reference
+def _reference_schema(golden_dir):
+    """Flattened configs and the model's state_dict shapes, as the unmodified reference produces them
+    (tests/golden/make_golden_schema.py)."""
+    return json.loads((golden_dir / 'reference_schema.json').read_text())
+
+
 @pytest.mark.parametrize('name,key', [('two_head_model', 'two_head'), ('midi_conformer', 'midi_conformer'),
                                       ('quant_two_head_model', 'quant_two_head')])
-def test_named_configs_match_reference_yaml(name, key):
-    flat = sconfig.flatten_config(f'/root/reference/configs/{name}.yaml', root='/root/reference')
+def test_named_configs_match_reference_yaml(name, key, golden_dir):
+    flat = _reference_schema(golden_dir)['configs'][key]        # configs/{name}.yaml through the reference's read_full_config
     mine = synth.named_config(key)
     for k, v in mine.items():
         if k in ('midi_prob_deviation', 'rest_threshold') and key == 'quant_two_head':
@@ -138,21 +144,17 @@ def test_state_dict_schema_and_strict_loading(tmp_path):
         sconfig.check_supported(dict(cfg, units_dim=768))
 
 
-@pytest.mark.reference
-def test_schema_matches_reference_module():
-    sys.path.insert(0, '/root/reference')
-    try:
-        from modules.model.Gmidi_conform import midi_conforms
-    finally:
-        sys.path.remove('/root/reference')
+def test_schema_matches_reference_module(golden_dir):
+    ref = _reference_schema(golden_dir)['state_dict_shapes']     # midi_conforms(two_head).state_dict()
     cfg = synth.named_config('two_head')
-    ref = midi_conforms({'midi_extractor_args': dict(cfg['midi_extractor_args']), 'units_dim': 80,
-                         'midi_num_bins': 128}).state_dict()
     mine = sconfig.model_param_shapes(cfg)
     assert set(ref) == set(mine)
     for k, v in ref.items():
-        assert tuple(v.shape) == tuple(mine[k]), k
-    ref.update(synth.fabricate_state_dict(cfg))      # and the fabricated weights load strictly
+        assert tuple(v) == tuple(mine[k]), k
+    fabricated = synth.fabricate_state_dict(cfg)     # and the fabricated weights have the reference's schema
+    assert set(fabricated) == set(ref)
+    for k, v in fabricated.items():
+        assert tuple(v.shape) == tuple(ref[k]), k
 
 
 # --------------------------------------------------------------------------- weight packing
@@ -281,14 +283,18 @@ def test_infer_sharded_gloo_world2():
 
 
 # --------------------------------------------------------------------------- drop-in alias
-def test_inference_package_is_the_drop_in():
+def test_inference_package_is_the_drop_in(tmp_path):
+    # a stand-in for the original project's own ``inference`` package, on the path behind this repository
+    original = tmp_path / 'original'
+    (original / 'inference').mkdir(parents=True)
+    (original / 'inference' / '__init__.py').write_text("raise ImportError('the original inference package was imported')\n")
     code = ("import inference, some_b200.plugin as p; "
             "assert inference.MIDIExtractionInference is p.MIDIExtractionInference; "
             "assert issubclass(inference.QuantizedMIDIExtractionInference, inference.BaseInference); "
             "assert inference.task_inference_mapping['training.MIDIExtractionTask'] == 'inference.MIDIExtractionInference'; "
             "print('ok')")
-    env = dict(os.environ, PYTHONPATH=f'{REPO}:/root/reference')
-    out = subprocess.run([sys.executable, '-c', code], capture_output=True, text=True, env=env, cwd='/tmp')
+    env = dict(os.environ, PYTHONPATH=os.pathsep.join([str(REPO), str(original)]))
+    out = subprocess.run([sys.executable, '-c', code], capture_output=True, text=True, env=env, cwd=tmp_path)
     assert out.returncode == 0 and 'ok' in out.stdout, out.stderr
 
 
